@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — headline benchmark of the render path (contract: see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A step = one frame of BASELINE config C2 (reference data/cover_scene.json objects, 800x600, 128 spp, depth 50,
@@ -38,7 +38,13 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="CPU time of the cpu_baseline sample of the GPU arm")
     ap.add_argument("--cpu-budget", type=float, default=150.0, help="--impl reference: CPU seconds for all warmup+steps renders")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's frame: it needs --impl ours")
+    return args
 
 
 def measured_peaks():
@@ -277,6 +283,25 @@ def sha256_of(a) -> str:
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
+DUMP_LIMIT_BYTES = 60 << 20     # array data; with the .npy headers a dump stays under 64 MB
+
+
+def dump_outputs(out_dir: str, frame) -> None:
+    """Write the RGB8 frame of the last timed step as <out_dir>/frame_rgb8.npy (float32 [H, W, 3], values 0..255), so that
+    two builds can be compared output for output. A frame above DUMP_LIMIT_BYTES (C5: 3840x2160) is written as a fixed,
+    seeded sample of its pixels, float32 [k, 3], with their row-major pixel indices in frame_pixel_index.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    f = np.asarray(frame, dtype=np.float32)
+    if f.nbytes > DUMP_LIMIT_BYTES:
+        px = f.reshape(-1, f.shape[-1])
+        k = DUMP_LIMIT_BYTES // (px.shape[1] * 4 + 8)
+        idx = np.sort(np.random.default_rng(0x5EED).choice(px.shape[0], k, replace=False))
+        np.save(os.path.join(out_dir, "frame_pixel_index.npy"), idx.astype(np.float64))
+        f = px[idx]
+    np.save(os.path.join(out_dir, "frame_rgb8.npy"), f)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -415,6 +440,8 @@ def run_ours(args):
         return
     # frame sanity: what we timed is the real image
     frame = rdr.frame.cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, frame)
     assert frame.shape == (h, w, 3) and frame.any()
     assert np.array_equal(frame, host_frame.numpy()), "resident and host-path frames differ"
     assert golden["status"] != "MISMATCH", f"frame differs from the oracle golden: {golden}"
