@@ -190,6 +190,35 @@ int rtb200_render_device_wait(rtb200_scene_handle h, rt_stats* stats);
 int rtb200_scene_release(rtb200_scene_handle h);
 int rtb200_scene_kernel_info(rtb200_scene_handle h, rt_kernel_info* out);
 
+/* Per-frame edits of a resident scene (animation, interactive camera) without a new upload. NULL fields are kept.
+ *   - camera and seed change host-side state only;
+ *   - spheres: exactly the uploaded count, same order (order is semantic). Centre, radius, material kind, albedo, param and
+ *     texture index may change. The host validates every new sphere with the rules of rtb200_scene_upload, copies the array
+ *     to the device once (64 B per sphere), and the device rebuilds what the closest-hit stage reads: exact geometry and
+ *     materials (every variant), the flat records (RT_VARIANT_BRUTE_FORCE) and, for the hierarchy, the leaf records and the
+ *     node boxes. The hierarchy's topology and recentring are those of the upload; boxes are recomputed with the builder's
+ *     own formulas (refit), so the frame is bit-identical to a fresh upload of the edited scene, but the tree gets looser as
+ *     spheres drift (rt_stats.nodes / clusters grow). Re-upload to rebuild it (DESIGN.md §4.6).
+ *   - refused, with the handle unchanged: a different count (RT_ERR_INVALID); a Light at a different set of indices
+ *     (RT_ERR_UNSUPPORTED: the kernel variant, light list and launch geometry were chosen from it); a sphere of the hierarchy
+ *     that leaves the upload's recentred f32 frame, i.e. non-finite or max|c-g|+|r| >= 1e15 (RT_ERR_UNSUPPORTED: re-upload);
+ *     spheres the upload put on the always-list may take any valid value. Also refused while asynchronous frames of the
+ *     handle are pending (RT_ERR_INVALID: call rtb200_render_device_wait first; they read the same scene arrays).
+ *   - every render enqueued after the call returns, on any stream, sees the edited scene. */
+typedef struct {
+    const rt_camera* camera;     /* NULL: keep */
+    const uint64_t*  seed;       /* NULL: keep */
+    const rt_sphere* spheres;    /* NULL: keep; else n_spheres == the uploaded count, same order */
+    uint64_t         n_spheres;
+} rt_scene_edit;
+int rtb200_scene_update(rtb200_scene_handle h, const rt_scene_edit* e);
+/* What the handle's closest-hit stage reads NOW, copied back from the device: the arrays and info[] of rtb200_debug_bvh.
+ * The flat records exist only on RT_VARIANT_BRUTE_FORCE handles (info[6] = 0 otherwise); RT_VARIANT_EXACT_F64 handles
+ * hold no hierarchy (info[0] = info[1] = 0). */
+int rtb200_scene_debug_bvh(rtb200_scene_handle h, double recentre[3], uint32_t info[8], float* nodes, uint64_t cap_nodes,
+                           float* leaf_rec, uint64_t cap_leaf_rec, uint32_t* leaf_id, uint64_t cap_leaf_id,
+                           uint32_t* always, uint64_t cap_always, float* flat, uint64_t cap_flat);
+
 /* load_texture_image — materials.rs:213-219, config.rs:36-47: decode a baseline JPEG file to RGB8 (host-side scene staging
  * helper for hosts without their own decoder; the reference uses the jpeg-decoder crate). *out_rgb8 is released with rtb200_free(). */
 int  rtb200_decode_jpeg_file(const char* path, uint8_t** out_rgb8, uint64_t* width, uint64_t* height);

@@ -150,6 +150,23 @@ uint32_t mode_of(uint32_t variant) {
     return variant == RT_VARIANT_EXACT_F64 ? MODE_EXACT : (variant == RT_VARIANT_BRUTE_FORCE ? MODE_BRUTE : MODE_TREE);
 }
 
+bool image_ok(const rt_image& im) {
+    if (!im.rgb8 || im.width == 0 || im.height == 0) return false;
+    if (im.width > (1ull << 20) || im.height > (1ull << 20)) return false;
+    return im.width * im.height * 3ull <= im.bytes;   // the callee reads width*height*3 bytes: the buffer must hold them
+}
+
+// The per-sphere rules of a scene (rtb200_scene_upload and rtb200_scene_update); tex_ok(t): texture t passes image_ok.
+template <typename TexOk>
+int validate_sphere(const rt_sphere& sp, uint64_t n_textures, TexOk tex_ok) {
+    if (sp.kind > RT_LIGHT) return fail(RT_ERR_INVALID, "unknown material kind");
+    if (sp.kind == RT_TEXTURE) {
+        if (sp.texture < 0 || (uint64_t)sp.texture >= n_textures) return fail(RT_ERR_INVALID, "texture index out of range");
+        if (!tex_ok(sp.texture)) return fail(RT_ERR_INVALID, "texture image is empty or smaller than width*height*3 bytes (rt_image.bytes)");
+    }
+    return RT_OK;
+}
+
 }  // namespace
 
 struct rtb200_scene_t {
@@ -178,6 +195,14 @@ struct rtb200_scene_t {
     uint32_t last_batches = 0, last_launches = 0;
     uint32_t pending_frames = 0;
     uint64_t h2d_bytes = 0;
+    // what rtb200_scene_update checks edits against (fixed at upload)
+    std::vector<uint32_t> light_ids;     // Light spheres, list order
+    std::vector<uint32_t> always_ids;    // spheres outside the hierarchy (MODE_TREE), increasing
+    std::vector<uint8_t> tex_ok;         // per texture: holds width*height*3 bytes
+    // refit state, allocated by the first sphere edit: ONE device allocation (sphere copy, maps, f64 slot boxes)
+    void* refit = nullptr;
+    RefitParams rp{};
+    cudaEvent_t written = nullptr;       // the last edit's device work; renders on other streams wait for it
 };
 
 extern "C" {
@@ -262,6 +287,8 @@ int rtb200_scene_release(rtb200_scene_handle h) {
             if (h->arena_cap <= (64u << 20) && cache.size() < 4) cache.push_back(DeviceCtx::Arena{h->arena, h->arena_cap});
             else cudaFree(h->arena);
         }
+        if (h->refit) cudaFree(h->refit);
+        if (h->written) cudaEventDestroy(h->written);
     }
     delete h;
     return RT_OK;
@@ -317,20 +344,12 @@ static int validate_scene(const rt_scene* s, uint32_t* n_lights_out) {
     if (s->n_spheres >= (1ull << 26)) return fail(RT_ERR_UNSUPPORTED, "2^26 or more spheres (list entries carry 27-bit ids)");
     if (s->n_spheres && !s->spheres) return fail(RT_ERR_INVALID, "spheres is null");
     if (s->n_textures && !s->textures) return fail(RT_ERR_INVALID, "textures is null");
-    auto image_ok = [](const rt_image& im) {
-        if (!im.rgb8 || im.width == 0 || im.height == 0) return false;
-        if (im.width > (1ull << 20) || im.height > (1ull << 20)) return false;
-        return im.width * im.height * 3ull <= im.bytes;   // the callee reads width*height*3 bytes: the buffer must hold them
-    };
     uint32_t n_lights = 0;
     for (uint64_t i = 0; i < s->n_spheres; ++i) {
         const rt_sphere& sp = s->spheres[i];
-        if (sp.kind > RT_LIGHT) return fail(RT_ERR_INVALID, "unknown material kind");
+        int rc = validate_sphere(sp, s->n_textures, [&](int32_t t) { return image_ok(s->textures[t]); });
+        if (rc != RT_OK) return rc;
         if (sp.kind == RT_LIGHT) ++n_lights;
-        if (sp.kind == RT_TEXTURE) {
-            if (sp.texture < 0 || (uint64_t)sp.texture >= s->n_textures) return fail(RT_ERR_INVALID, "texture index out of range");
-            if (!image_ok(s->textures[sp.texture])) return fail(RT_ERR_INVALID, "texture image is empty or smaller than width*height*3 bytes (rt_image.bytes)");
-        }
     }
     if (n_lights >= 10) return fail(RT_ERR_UNSUPPORTED, "10 or more lights: the reference's light recursion (raytracer.rs:99-114) does not terminate when n_lights * 0.1 >= 1");
     if (s->sky.mode > RT_SKY_TEXTURE) return fail(RT_ERR_INVALID, "unknown sky mode");
@@ -394,6 +413,10 @@ static int scene_upload_records(const rt_scene* s, const rt_options& opts, uint3
     }
     std::vector<uint32_t> lights;
     for (uint32_t i = 0; i < n; ++i) if (s->spheres[i].kind == RT_LIGHT) lights.push_back(i);
+    h->light_ids = lights;
+    h->always_ids = R.always;
+    h->tex_ok.resize(s->n_textures);
+    for (uint64_t t = 0; t < s->n_textures; ++t) h->tex_ok[t] = image_ok(s->textures[t]);
     lights.push_back(0);
     upload_array(h, lights.data(), lights.size() * 4, (void**)&tp.lights);
     upload_array(h, nullptr, 16, (void**)&h->err);   // zero-filled error counters
@@ -491,6 +514,126 @@ int rtb200_scene_kernel_info(rtb200_scene_handle h, rt_kernel_info* out) {
     return RT_OK;
 }
 
+// ---- resident scene edits ------------------------------------------------------------------------------
+// Host side of rtb200_scene_update: O(n) validation, ONE host->device copy of the rt_sphere array, then the device rebuilds
+// the records (rtb200_refit.cu). Nothing on the device is written before the whole edit has been validated.
+static int validate_edit(const rtb200_scene_t* h, const rt_sphere* sp, uint64_t n) {
+    if (n != h->tp.n) return fail(RT_ERR_INVALID, "rt_scene_edit.n_spheres must equal the uploaded sphere count");
+    const double g[3] = {h->tp.gx, h->tp.gy, h->tp.gz};
+    size_t li = 0, ai = 0;
+    for (uint64_t i = 0; i < n; ++i) {
+        const rt_sphere& s = sp[i];
+        int rc = validate_sphere(s, h->tex_ok.size(), [&](int32_t t) { return h->tex_ok[t] != 0; });
+        if (rc != RT_OK) return rc;
+        const bool was_light = li < h->light_ids.size() && h->light_ids[li] == i;
+        li += was_light;
+        if ((s.kind == RT_LIGHT) != was_light)
+            return fail(RT_ERR_UNSUPPORTED, "the Light spheres must stay at the uploaded indices (kernel variant, light list and launch geometry were chosen from them): re-upload");
+        if (h->mode != MODE_TREE) continue;
+        const bool always = ai < h->always_ids.size() && h->always_ids[ai] == i;
+        ai += always;
+        if (!always && !rtbvh::in_f32_frame(s, g))
+            return fail(RT_ERR_UNSUPPORTED, "sphere " + std::to_string(i) + " of the hierarchy leaves the upload's recentred f32 frame (non-finite, or max|c-g|+|r| >= 1e15): re-upload");
+    }
+    return RT_OK;
+}
+
+// First sphere edit of a handle: one allocation for the sphere copy and the maps of the refit, which are built on the device.
+static int refit_init(rtb200_scene_t* h) {
+    const TraceParams& tp = h->tp;
+    const size_t n = tp.n, nn = tp.n_nodes;
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b_sp = al(n * sizeof(rt_sphere)), b_slot = al(n * 4), b_node = al(nn * 4), b_box = al(nn * 8 * 6 * sizeof(double));
+    CU(cudaMalloc(&h->refit, b_sp + b_slot + 2 * b_node + b_box + 256));
+    char* b = (char*)h->refit;
+    RefitParams& p = h->rp;
+    p.sp = (const rt_sphere*)b;                     b += b_sp;
+    p.slot_of = (uint32_t*)b;                       b += b_slot;
+    p.parent = (uint32_t*)b;                        b += b_node;
+    p.level = (uint32_t*)b;                         b += b_node;
+    p.box64 = (double*)b;
+    p.n = tp.n; p.n_nodes = tp.n_nodes; p.n_leaves = tp.n_leaves;
+    p.gx = tp.gx; p.gy = tp.gy; p.gz = tp.gz;
+    p.geo = (double4*)tp.geo; p.mat = (DevMat*)tp.mat;
+    p.flat = h->mode == MODE_BRUTE ? (float*)tp.filt : nullptr;
+    p.leaf_rec = (float*)tp.leaf_rec; p.leaf_id = tp.leaf_id; p.nodes = (float*)tp.nodes;
+    cudaStream_t st = h->ctx->stream;
+    CU(cudaMemsetAsync(p.slot_of, 0xff, n * 4, st));
+    CU(cudaMemsetAsync(p.parent, 0xff, nn * 4, st));
+    CU(launch_refit_maps(p, st));
+    CU(cudaEventCreateWithFlags(&h->written, cudaEventDisableTiming));
+    return RT_OK;
+}
+
+static int refit(rtb200_scene_t* h, const rt_sphere* sp) {
+    DeviceCtx* ctx = h->ctx;
+    CU(cudaSetDevice(h->device));
+    if (!h->refit) {
+        int rc = refit_init(h);
+        if (rc != RT_OK) {
+            if (h->refit) cudaFree(h->refit);
+            if (h->written) cudaEventDestroy(h->written);
+            h->refit = nullptr; h->written = nullptr;
+            return rc;
+        }
+    }
+    // through the context's pinned staging buffer (like an upload): the caller may reuse its array as soon as we return
+    const size_t bytes = (size_t)h->tp.n * sizeof(rt_sphere);
+    CU(cudaEventSynchronize(ctx->staging_free));
+    CU(ctx->staging.ensure(bytes));
+    memcpy(ctx->staging.p, sp, bytes);
+    CU(cudaMemcpyAsync((void*)h->rp.sp, ctx->staging.p, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaEventRecord(ctx->staging_free, ctx->stream));
+    CU(launch_refit(h->rp, h->tp.depth, ctx->stream));
+    CU(cudaEventRecord(h->written, ctx->stream));
+    return RT_OK;
+}
+
+int rtb200_scene_update(rtb200_scene_handle h, const rt_scene_edit* e) {
+  return guarded([&]() -> int {
+    if (!h || !e) return fail(RT_ERR_INVALID, "null argument");
+    DeviceRestore restore;
+    std::lock_guard<std::recursive_mutex> lk(h->ctx->mu);
+    if (h->pending_frames) return fail(RT_ERR_INVALID, "asynchronous frames of this scene are in flight and read its arrays: call rtb200_render_device_wait first");
+    if (e->spheres) {
+        int rc = validate_edit(h, e->spheres, e->n_spheres);
+        if (rc != RT_OK) return rc;
+        if (h->tp.n && (rc = refit(h, e->spheres)) != RT_OK) return rc;
+    }
+    if (e->camera) h->tp.cam = *e->camera;
+    if (e->seed) { h->tp.key0 = (uint32_t)*e->seed; h->tp.key1 = (uint32_t)(*e->seed >> 32); }
+    return RT_OK;
+  });
+}
+
+int rtb200_scene_debug_bvh(rtb200_scene_handle h, double recentre[3], uint32_t info[8], float* nodes, uint64_t cap_nodes,
+                           float* leaf_rec, uint64_t cap_leaf_rec, uint32_t* leaf_id, uint64_t cap_leaf_id,
+                           uint32_t* always, uint64_t cap_always, float* flat, uint64_t cap_flat) {
+  return guarded([&]() -> int {
+    if (!h || !info) return fail(RT_ERR_INVALID, "null argument");
+    DeviceRestore restore;
+    std::lock_guard<std::recursive_mutex> lk(h->ctx->mu);
+    CU(cudaSetDevice(h->device));
+    const TraceParams& tp = h->tp;
+    const uint32_t n_pairs = h->mode == MODE_BRUTE ? tp.n_pairs : 0u;
+    if (recentre) { recentre[0] = tp.gx; recentre[1] = tp.gy; recentre[2] = tp.gz; }
+    info[0] = tp.n_nodes; info[1] = tp.n_leaves; info[2] = tp.depth; info[3] = (uint32_t)rtbvh::kLeafK; info[4] = tp.n_always;
+    info[5] = (uint32_t)rtbvh::kNodeFloats; info[6] = n_pairs; info[7] = 0;
+    cudaStream_t st = h->ctx->stream;   // after the handle's edits
+    auto get = [&](void* dst, uint64_t cap, const void* src, uint64_t count) -> cudaError_t {
+        const uint64_t k = std::min(cap, count);
+        return dst && k ? cudaMemcpyAsync(dst, src, k * 4, cudaMemcpyDeviceToHost, st) : cudaSuccess;
+    };
+    CU(get(nodes, cap_nodes, tp.nodes, (uint64_t)tp.n_nodes * rtbvh::kNodeFloats));
+    CU(get(leaf_rec, cap_leaf_rec, tp.leaf_rec, (uint64_t)tp.n_leaves * rtbvh::kLeafK * 4));
+    CU(get(leaf_id, cap_leaf_id, tp.leaf_id, (uint64_t)tp.n_leaves * rtbvh::kLeafK));
+    CU(get(always, cap_always, tp.always, tp.n_always));
+    CU(get(flat, cap_flat, tp.filt, (uint64_t)n_pairs * 8));
+    CU(cudaStreamSynchronize(st));
+    return RT_OK;
+  });
+}
+
 // Enqueue one frame on `stream_in` (or the context's stream) without waiting for it.
 static int render_enqueue(rtb200_scene_handle h, void* dev_rgb8, void* dev_linear_f32, void* stream_in, int set) {
     if (!h) return fail(RT_ERR_INVALID, "null scene handle");
@@ -498,7 +641,10 @@ static int render_enqueue(rtb200_scene_handle h, void* dev_rgb8, void* dev_linea
     DeviceCtx::WorkSet& W = ctx->ws[set & 1];
     CU(cudaSetDevice(h->device));
     cudaStream_t st = stream_in ? (cudaStream_t)stream_in : ctx->stream;
-    if (st != ctx->stream) CU(cudaStreamWaitEvent(st, ctx->staging_free, 0));   // the scene upload ran on the context's stream
+    if (st != ctx->stream) {   // the scene upload and edits ran on the context's stream
+        CU(cudaStreamWaitEvent(st, ctx->staging_free, 0));
+        if (h->written) CU(cudaStreamWaitEvent(st, h->written, 0));
+    }
     TraceParams tp = h->tp;
     h->last_stream = st; h->last_set = set & 1; h->last_batches = 0; h->last_launches = 0;
     if (h->n_streams < 2 && (h->n_streams == 0 || h->streams[0] != st)) h->streams[h->n_streams++] = st;

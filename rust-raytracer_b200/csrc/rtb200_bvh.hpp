@@ -78,6 +78,16 @@ inline bool sphere_record(double x, double y, double z, double r2, float rec[4])
     return std::isfinite(rec[0]) && std::isfinite(rec[1]) && std::isfinite(rec[2]) && std::isfinite(nkd) && c2 < 1e30;
 }
 
+// Whether sphere `sp` lives in the hierarchy of the frame recentred on g (else it goes to the always-list): finite, and
+// max|c-g| + |r| < 1e15. rtb200_scene_update applies the same test to edited spheres of the hierarchy.
+inline bool in_f32_frame(const rt_sphere& sp, const double g[3]) {
+    const double c[3] = {sp.center.x - g[0], sp.center.y - g[1], sp.center.z - g[2]};
+    const double r = std::fabs(sp.radius);
+    const bool fin = std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]) && std::isfinite(r);
+    const double ext = fin ? std::max(std::max(std::fabs(c[0]), std::fabs(c[1])), std::fabs(c[2])) + r : INFINITY;
+    return fin && ext < 1e15;
+}
+
 struct Box {
     double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
     void grow(const Box& o) { for (int a = 0; a < 3; ++a) { lo[a] = std::min(lo[a], o.lo[a]); hi[a] = std::max(hi[a], o.hi[a]); } }
@@ -104,11 +114,9 @@ public:
         // primitives of the hierarchy: spheres that live in the f32 frame; the rest is tested for every ray
         for (uint32_t i = 0; i < n; ++i) {
             const rt_sphere& sp = s_->spheres[i];
+            if (!in_f32_frame(sp, R_.g)) { R_.always.push_back(i); continue; }
             double c[3] = {sp.center.x - R_.g[0], sp.center.y - R_.g[1], sp.center.z - R_.g[2]};
             const double r = std::fabs(sp.radius);
-            const bool fin = std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]) && std::isfinite(r);
-            const double ext = fin ? std::max(std::max(std::fabs(c[0]), std::fabs(c[1])), std::fabs(c[2])) + r : INFINITY;
-            if (!fin || !(ext < 1e15)) { R_.always.push_back(i); continue; }
             Box b;
             for (int a = 0; a < 3; ++a) { b.lo[a] = c[a] - r; b.hi[a] = c[a] + r; }
             prim_box_.push_back(b);

@@ -96,6 +96,24 @@ struct ResolveParams {
     uint8_t* out_rgb8;     // [npix_local][3] or null
 };
 
+// On-device refit of a resident scene after a sphere edit (rtb200_scene_update, rtb200_refit.cu). The topology (child refs,
+// leaf_id, always-list) and the recentring g are those of the upload; everything else is rebuilt from `sp`.
+struct RefitParams {
+    const rt_sphere* sp;         // n new spheres (device copy of the caller's array)
+    uint32_t n, n_nodes, n_leaves;
+    double gx, gy, gz;
+    double4* geo;                // n
+    DevMat*  mat;                // n
+    float*   flat;               // n_pairs * 8, or null (only MODE_BRUTE handles hold flat records)
+    float*   leaf_rec;           // n_leaves * kLeafK * 4
+    const uint32_t* leaf_id;     // n_leaves * kLeafK
+    float*   nodes;              // n_nodes * kNodeVec * 4: the boxes are rewritten, child[] is read
+    uint32_t* slot_of;           // n: sphere -> leaf slot (0xffffffff: not in the hierarchy)
+    uint32_t* parent;            // n_nodes: parent node (root: 0xffffffff)
+    uint32_t* level;             // n_nodes: wide level, root = 1 (emit_wide's numbering)
+    double*  box64;              // n_nodes * 8 * 6: exact f64 box of every child slot {lo xyz, hi xyz} before inflation
+};
+
 struct KernelInfo { int registers, max_threads, const_bytes, local_bytes; char name[96]; };
 
 size_t wavefront_smem_bytes(const TraceParams& p, uint32_t mode, uint32_t smem_mask);
@@ -103,6 +121,9 @@ cudaError_t launch_wavefront(const TraceParams& p, uint32_t mode, int grid, size
 int wavefront_max_ctas_per_sm(uint32_t mode, bool lights, size_t smem, int minb);
 cudaError_t wavefront_info(uint32_t mode, bool lights, int minb, KernelInfo* out);
 cudaError_t launch_resolve(const ResolveParams& p, cudaStream_t st);
+// refit: maps once per handle (slot_of / parent / level), then per edit the sphere pass and one node pass per level, deepest first
+cudaError_t launch_refit_maps(const RefitParams& p, cudaStream_t st);
+cudaError_t launch_refit(const RefitParams& p, uint32_t depth, cudaStream_t st);
 
 // single-thread probes of the device routines (known-answer tests)
 cudaError_t probe_sphere_hit(const double* in /*12*/, double* out /*9*/, cudaStream_t st);

@@ -96,6 +96,10 @@ class rt_kernel_info(C.Structure):
         return d
 
 
+class rt_scene_edit(C.Structure):
+    _fields_ = [("camera", C.POINTER(rt_camera)), ("seed", C.POINTER(C.c_uint64)), ("spheres", C.POINTER(rt_sphere)), ("n_spheres", C.c_uint64)]
+
+
 assert C.sizeof(rt_sphere) == 64
 
 # every symbol include/rtb200.h declares (tests check that the library exports all of them)
@@ -106,6 +110,7 @@ ABI_SYMBOLS = [
     "rtb200_probe_sky", "rtb200_probe_get_ray", "rtb200_probe_rng", "rtb200_probe_quantise",
     "rtb200_decode_jpeg_file", "rtb200_free", "rtb200_render_device_async", "rtb200_render_device_wait",
     "rtb200_debug_bvh", "rtb200_probe_sphere_uv", "rtb200_device_count", "rtb200_render_rgb8_multi", "rtb200_scene_kernel_info",
+    "rtb200_scene_update", "rtb200_scene_debug_bvh",
 ]
 
 _lib = None
@@ -149,6 +154,8 @@ def lib() -> C.CDLL:
     L.rtb200_device_count.restype = C.c_int
     L.rtb200_render_rgb8_multi.argtypes = [C.POINTER(rt_scene), C.POINTER(rt_options), C.c_int32, C.c_void_p, C.POINTER(rt_stats)]
     L.rtb200_scene_kernel_info.argtypes = [C.c_void_p, C.POINTER(rt_kernel_info)]
+    L.rtb200_scene_update.argtypes = [C.c_void_p, C.POINTER(rt_scene_edit)]
+    L.rtb200_scene_debug_bvh.argtypes = [C.c_void_p] + L.rtb200_debug_bvh.argtypes[1:]
     _lib = L
     return L
 
@@ -337,14 +344,18 @@ def load_scene(path: str, base_dir: Optional[str] = None) -> Scene:
 
 def bvh_records(scene: "Scene") -> dict:
     """Host-side diagnostic: the hierarchy the closest-hit stage traverses (no GPU needed). See rtb200_debug_bvh."""
-    n = scene.n_spheres
+    return _bvh_dict(lambda *a: lib().rtb200_debug_bvh(C.byref(scene.c), *a), scene.n_spheres)
+
+
+def _bvh_dict(debug_bvh, n: int) -> dict:
+    """Calls debug_bvh(recentre, info, nodes, cap, leaf_rec, cap, leaf_id, cap, always, cap, flat, cap) twice (sizes, then arrays)."""
     g = (C.c_double * 3)(); info = (C.c_uint32 * 8)()
-    _check(lib().rtb200_debug_bvh(C.byref(scene.c), g, info, None, 0, None, 0, None, 0, None, 0, None, 0))
+    _check(debug_bvh(g, info, None, 0, None, 0, None, 0, None, 0, None, 0))
     n_nodes, n_leaves, depth, k, n_always, fpn, n_pairs, _ = (int(x) for x in info)
     nodes = np.zeros(max(n_nodes * fpn, 1), np.float32); rec = np.zeros(max(n_leaves * k * 4, 1), np.float32)
     ids = np.zeros(max(n_leaves * k, 1), np.uint32); always = np.zeros(max(n_always, 1), np.uint32); flat = np.zeros(max(n_pairs * 8, 1), np.float32)
-    _check(lib().rtb200_debug_bvh(C.byref(scene.c), g, info, nodes.ctypes.data, nodes.size, rec.ctypes.data, rec.size, ids.ctypes.data, ids.size,
-                                  always.ctypes.data, always.size, flat.ctypes.data, flat.size))
+    _check(debug_bvh(g, info, nodes.ctypes.data, nodes.size, rec.ctypes.data, rec.size, ids.ctypes.data, ids.size,
+                     always.ctypes.data, always.size, flat.ctypes.data, flat.size))
     nd = nodes[: n_nodes * fpn].reshape(n_nodes, fpn)
     return {"n_nodes": n_nodes, "n_leaves": n_leaves, "depth": depth, "leaf_size": k, "recentre": np.array(g[:]), "n": n,
             "lo": nd[:, :24].reshape(n_nodes, 3, 8), "hi": nd[:, 24:48].reshape(n_nodes, 3, 8), "child": nd[:, 48:56].view(np.uint32),
@@ -413,6 +424,26 @@ class ResidentScene:
         st = rt_stats()
         _check(lib().rtb200_render_device_wait(self.h, C.byref(st)))
         return st.as_dict()
+
+    def update(self, spheres=None, camera: Optional[rt_camera] = None, seed: Optional[int] = None):
+        """rtb200_scene_update: edit the resident scene for the next frames (None keeps a field). `spheres` is a
+        :class:`Scene` (its sphere list) or a ctypes ``rt_sphere`` array with the uploaded count, in the same order."""
+        e = rt_scene_edit()
+        if spheres is not None:
+            if isinstance(spheres, Scene):
+                e.spheres, e.n_spheres = spheres.c.spheres, spheres.c.n_spheres
+            else:
+                e.spheres, e.n_spheres = C.cast(spheres, C.POINTER(rt_sphere)), len(spheres)
+        if camera is not None:
+            e.camera = C.pointer(camera)
+        if seed is not None:
+            e.seed = C.pointer(C.c_uint64(int(seed)))
+        _check(lib().rtb200_scene_update(self.h, C.byref(e)))
+
+    def bvh_records(self) -> dict:
+        """What the closest-hit stage of this handle reads now (after any update), copied back from the device;
+        the dict of :func:`bvh_records`. ``flat`` is empty unless the handle renders RT_VARIANT_BRUTE_FORCE."""
+        return _bvh_dict(lambda *a: lib().rtb200_scene_debug_bvh(self.h, *a), int(self.scene.c.n_spheres))
 
     def kernel_info(self) -> dict:
         ki = rt_kernel_info()
